@@ -1,7 +1,11 @@
 #!/usr/bin/env python
 """Benchmark of the cascade-MVS depth hot path on B200 (contract: task prompt §④).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned (depth_l, confidence_l; at N > 1 also
+depth_0_all_ranks, the gathered depth maps of that step) as DIR/<name>.npy, float32.  Inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.
 
 A *step* is one `CascadeMVSNet.forward` (FeatureNet + three cascade stages) over
 one batch of synthetic DTU-shaped views per GPU: BASELINE.json configs[1] —
@@ -171,6 +175,14 @@ def best_cpu_threads(cores):
     return best_t
 
 
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> tensor; written as out_dir/<name>.npy in float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy().astype(np.float32))
+
+
 def time_cpu_port(steps, warmup, threads, want_result=False):
     fwd = cpu_port_forward_factory(threads)
     for _ in range(warmup):
@@ -194,7 +206,9 @@ def run_reference_arm(args, rank):
     avail = len(os.sched_getaffinity(0))
     cores = best_cpu_threads(avail)
     steps = max(1, args.steps)
-    med, total = time_cpu_port(steps, max(1, min(args.warmup, 2)), cores)
+    med, total, res = time_cpu_port(steps, max(1, min(args.warmup, 2)), cores, want_result=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     value = steps / total
     sample = (f"{steps} full forwards of the cfg2 workload (640x512, V=3, D=48/32/8, B=1) on "
               f"{cores} torch threads (fastest of 4..{avail} available; more threads are slower); "
@@ -421,7 +435,11 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-sharded-configs", action="store_true",
                     help="skip the cfg4 / cfg5 sharded-batch runs at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -580,8 +598,19 @@ def main():
     if sampler:
         sampler.start()
     n0 = _lib.launch_count()
-    ms_total = timed(run_resident, K)
+    last = []
+    ms_total = timed(lambda steps: last.append(run_resident(steps)), K)
     launches = _lib.launch_count() - n0
+    if args.dump_outputs:
+        # copied now: the e2e and latency runs below replay into the same result buffers
+        dumped = {k: v.cpu() for k, v in last[0].items()}
+        if world > 1:
+            # gathered[] holds each chunk of steps k0..K-1 rank by rank
+            k0 = (K - 1) // GATHER_EVERY * GATHER_EVERY
+            rows = [(world * k0 + r * (K - k0) + K - 1 - k0) * B for r in range(world)]
+            dumped["depth_0_all_ranks"] = torch.stack([gathered[i:i + B] for i in rows]).cpu()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, dumped)
     if graphed is not None:      # graph replays launch the captured libcasmvs kernels
         launches += graphed.kernels_per_replay * K
     run_e2e(max(3, args.warmup))     # copy engines / PCIe links idled during the resident timing

@@ -6,8 +6,8 @@ is nn.Module code).  Each function cites the reference file:line it follows
 (paths relative to /root/reference).  It uses the same torch primitives in the
 same order as the reference, so on CPU it is bit-identical to the reference
 run in this container; that is pinned by ``tests/golden/*.npz`` (generated from
-the REAL reference by ``oracle/make_golden.py``) and by
-``tests/test_oracle_vs_reference.py`` when /root/reference is present.
+the REAL reference by ``oracle/make_golden.py``), which ``tests/test_oracle_golden.py``
+and ``tests/test_oracle_vs_reference.py`` compare against.
 
 Parity status: the reference ships no tests / golden vectors of its own
 ("parity unpinned" by the reference, SURVEY.md §8c); the pins above are outputs

@@ -9,6 +9,8 @@ outputs of the reference itself are the pins for both the oracle restatement
 every array needed to replay a case is stored inline except model weights, which
 are regenerated from a seed (a checksum guards against RNG drift).
 """
+import hashlib
+import json
 import os
 import sys
 
@@ -23,6 +25,9 @@ from casmvsnet_pl_b200.models.mvsnet import CascadeMVSNet      # noqa: E402
 from oracle import ref_loader                                  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
+# ATen and oneDNN split CPU reductions by thread count, so the bits of a fixture depend on it;
+# the bit-exact tests run with the same count
+GOLDEN_THREADS = 8
 
 
 def seeded_state_dict(n_depths, interval_ratios, G, seed):
@@ -56,7 +61,7 @@ def save(name, **arrays):
 
 
 def main():
-    torch.set_num_threads(8)
+    torch.set_num_threads(GOLDEN_THREADS)
     mvsnet, modules, abn = ref_loader.load_reference_models()
 
     # ---- a1 homo_warp: stress geometry + behind-camera branch ------------------
@@ -168,6 +173,71 @@ def main():
         res = ref(imgs, pm, dmin, dint)
     save("cascade_var_tensorparams_96x64", sd_checksum=np.float64(sd_checksum(sd)),
          init_depth_min=dmin, depth_interval=dint, **{k: v for k, v in res.items()})
+    reference_checks()
+
+
+def predict_depth_inputs():
+    """Seeded inputs of the predict_depth fixture: stress pose, one source view behind the
+    camera, per-pixel hypotheses."""
+    g = torch.Generator().manual_seed(9)
+    feats = torch.randn(2, 4, 16, 16, 24, generator=g)
+    pms = synth.projection_matrices(4, W=96, H=64, stress=True, behind_view=3)[:, 1]
+    pms = pms.unsqueeze(0).expand(2, -1, -1, -1).contiguous()
+    dv = 430.0 + 5.3 * torch.arange(16).float().reshape(1, 16, 1, 1) + torch.rand(2, 16, 16, 24, generator=g)
+    return feats, pms, dv
+
+
+def feature_pyramid_input():
+    return torch.randn(2, 3, 64, 96, generator=torch.Generator().manual_seed(2))
+
+
+def sample_index(n, k=1024):
+    """Fixed, seeded positions at which a fixture stores the values of a large output."""
+    return torch.randperm(n, generator=torch.Generator().manual_seed(0))[:k]
+
+
+def tensor_digest(t):
+    """SHA-256 of a float32 tensor's values in logical order: equal digests <=> torch.equal."""
+    return np.frombuffer(hashlib.sha256(t.contiguous().numpy().tobytes()).digest(), np.uint8)
+
+
+def reference_checks():
+    """Fixtures of tests/test_oracle_vs_reference.py and the state-dict layout of
+    tests/test_api_contract.py: the reference's predict_depth and feature pyramid on seeded
+    inputs (the pyramid as a digest of each level plus a sample of its values)."""
+    feats, pms, dv = predict_depth_inputs()
+    out = {}
+    for G in (1, 4):
+        sd = seeded_state_dict((8, 32, 48), (1, 2, 4), G, seed=5)
+        ref = ref_loader.make_reference_model((8, 32, 48), (1, 2, 4), G)
+        ref.load_state_dict(sd)
+        with torch.no_grad():
+            d, c = ref.predict_depth(feats, pms, dv, ref.cost_reg_1)
+        out.update({f"G{G}/sd_checksum": np.float64(sd_checksum(sd)), f"G{G}/depth": d,
+                    f"G{G}/confidence": c})
+    save("reference_predict_depth", **out)
+
+    sd = seeded_state_dict((8, 32, 48), (1, 2, 4), 1, seed=2)
+    ref = ref_loader.make_reference_model((8, 32, 48), (1, 2, 4), 1)
+    ref.load_state_dict(sd)
+    with torch.no_grad():
+        pyr = ref.feature(feature_pyramid_input())
+    out = {"sd_checksum": np.float64(sd_checksum(sd))}
+    for k, v in pyr.items():
+        out.update({f"{k}/shape": np.array(v.shape), f"{k}/sha256": tensor_digest(v),
+                    f"{k}/sample": v.flatten()[sample_index(v.numel())]})
+    save("reference_feature_pyramid", **out)
+
+    # {"<num_groups>": [[key, shape, dtype], ...]} in state-dict order, one entry per line
+    groups = []
+    for G in (1, 8):
+        sd = ref_loader.make_reference_model((8, 32, 48), (1, 2, 4), G).state_dict()
+        rows = [json.dumps([k, list(v.shape), str(v.dtype).replace("torch.", "")]) for k, v in sd.items()]
+        groups.append(f'"{G}": [\n' + ",\n".join(rows) + "\n]")
+    path = os.path.join(OUT, "reference_state_dict.json")
+    with open(path, "w") as f:
+        f.write("{\n" + ",\n".join(groups) + "\n}\n")
+    print(f"reference_state_dict: {os.path.getsize(path) / 1024:.0f} KiB")
 
 
 if __name__ == "__main__":

@@ -2,8 +2,8 @@
 
 Only usable in the build container (``/root/reference`` does not exist on the
 GPU box).  It is used by ``oracle/make_golden.py`` to generate the committed
-golden vectors and by ``tests/test_oracle_vs_reference.py`` (skipped when the
-reference tree is absent) to pin the restatement in ``oracle/casmvs_oracle.py``.
+golden vectors that pin the restatement in ``oracle/casmvs_oracle.py``; the
+tests read only those vectors.
 
 The reference imports two third-party packages that are neither installed nor
 vendored (SURVEY.md §8c): ``inplace_abn`` (README.md:28, unpinned) and

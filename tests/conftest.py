@@ -24,6 +24,18 @@ def golden():
     return load
 
 
+@pytest.fixture
+def golden_threads():
+    """CPU results are bit-exact only at the torch thread count the golden vectors were
+    generated with (oracle/make_golden.py), whatever the machine's core count."""
+    import torch
+    from oracle.make_golden import GOLDEN_THREADS
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.fixture(autouse=True)
 def _inference_mode_for_gpu_tests(request):
     """The engine is forward-only and refuses to run with grad enabled on parameters that

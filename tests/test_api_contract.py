@@ -1,6 +1,7 @@
 """Drop-in boundary (SURVEY.md §8b): constructor, attributes, state-dict keys and
 the no-CPU-fallback rule.  CPU only."""
 import inspect
+import json
 import os
 
 import pytest
@@ -9,7 +10,6 @@ import torch
 from casmvsnet_pl_b200 import ABN, InPlaceABN, _lib, synth
 from casmvsnet_pl_b200.models import modules as M
 from casmvsnet_pl_b200.models.mvsnet import CascadeMVSNet, CostRegNet, FeatureNet
-from oracle import ref_loader
 
 
 def test_reference_import_path_resolves():
@@ -50,15 +50,18 @@ def test_state_dict_has_206_reference_keys():
         assert tuple(sd[k].shape) == shape
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="/root/reference absent")
 @pytest.mark.parametrize("G", [1, 8])
 def test_state_dict_equals_reference(G):
-    ref = ref_loader.make_reference_model((8, 32, 48), (1, 2, 4), G)
+    """Keys, shapes and dtypes of the reference's state dict (oracle/make_golden.py ->
+    tests/golden/reference_state_dict.json), in order, and a strict load of that layout."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    with open(os.path.join(root, "tests", "golden", "reference_state_dict.json")) as f:
+        layout = json.load(f)[str(G)]
+    a = {k: torch.zeros(shape, dtype=getattr(torch, dtype)) for k, shape, dtype in layout}
     ours = CascadeMVSNet(num_groups=G, norm_act=ABN)
-    a, b = ref.state_dict(), ours.state_dict()
+    b = ours.state_dict()
     assert list(a) == list(b)
-    assert all(a[k].shape == b[k].shape for k in a)
-    ref.load_state_dict(b, strict=True)
+    assert all(a[k].shape == b[k].shape and a[k].dtype == b[k].dtype for k in a)
     ours.load_state_dict(a, strict=True)
 
 

@@ -6,6 +6,8 @@ import torch
 
 from oracle import casmvs_oracle as O
 
+pytestmark = pytest.mark.usefixtures("golden_threads")
+
 
 def test_homo_warp_bit_exact(golden):
     g = golden("homo_warp")

@@ -68,6 +68,9 @@ SIGNATURES = {
     "casmvs_bias_lrelu_nhwc": (c_int, [c_void_p, c_void_p, c_float, c_size_t, c_int, c_void_p]),
     "casmvs_normalize_u8_fwd": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, POINTER(c_float),
                                         POINTER(c_float), c_void_p]),
+    "casmvs_resize_u8_fwd": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int,
+                                     c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int,
+                                     c_void_p]),
     "casmvs_warp_cost_bwd": (c_int, [c_void_p] * 5 + [c_int] * 7 + [c_void_p]),
     "casmvs_conv3d_wgrad": (c_int, [c_void_p] * 3 + [c_int] * 10 + [c_void_p]),
     "casmvs_regress_bwd": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p] + [c_int] * 4 + [c_void_p]),

@@ -9,6 +9,10 @@ Host-side Python like the reference's (it is data plumbing, not arithmetic on th
   pyramid_proj_mats            reference datasets/dtu.py:52-75 (K[R|t] per level, fine -> coarse,
                                intrinsics doubled per finer level, optional test-mode rescale)
   relative_proj_mats           reference datasets/dtu.py:181-186 (src_proj @ inv(ref_proj), rows 0..2)
+  pil_bilinear_coeffs /        PIL.Image.resize(img_wh, Image.BILINEAR) of the data sets' network
+  resize_images                input (datasets/dtu.py:159-162, tanks.py, blendedmvs.py:162-163),
+                               bit-exact: PIL's fixed-point taps built here in float64, the
+                               integer passes on the GPU by casmvs_resize_u8_fwd
   normalize_images             reference datasets/dtu.py:130-137 (ToTensor + ImageNet Normalize):
                                uint8 HWC images are uploaded AS BYTES (4x less H2D traffic than
                                fp32) and converted + normalised + re-laid-out to planar fp32 on the
@@ -20,6 +24,8 @@ Host-side Python like the reference's (it is data plumbing, not arithmetic on th
 """
 from __future__ import annotations
 
+import functools
+import math
 import os
 import re
 import sys
@@ -157,6 +163,79 @@ def normalize_images(images_u8, device=None, out=None):
         _lib.check(_lib.load().casmvs_normalize_u8_fwd(
             ctypes.c_void_p(t.data_ptr()), ctypes.c_void_p(out.data_ptr()), N, H, W, mean, std, st),
             "normalize_u8")
+    return out
+
+
+@functools.lru_cache(maxsize=64)
+def pil_bilinear_coeffs(in_size, out_size):
+    """PIL's fixed-point BILINEAR resampling coefficients for one axis in_size -> out_size
+    (Pillow's precompute_coeffs + normalize_coeffs_8bpc, in float64 like its C code) ->
+    (xmin (out_size,) int32, taps (out_size, k) int32).  Output index o reads input
+    xmin[o] + j with weight taps[o, j] / 2**22; unused trailing taps are 0.  The arrays are
+    shared by later calls with the same sizes: do not modify them."""
+    in_size, out_size = int(in_size), int(out_size)
+    if in_size <= 0 or out_size <= 0:
+        raise ValueError(f"pil_bilinear_coeffs: sizes must be positive ({in_size} -> {out_size})")
+    scale = in_size / out_size
+    fs = max(scale, 1.0)
+    support = fs                               # bilinear support 1.0, widened when downscaling
+    ss = 1.0 / fs
+    xmin = np.zeros(out_size, np.int32)
+    taps = np.zeros((out_size, int(math.ceil(support)) * 2 + 1), np.int32)   # PIL's ksize
+    k = 1
+    for o in range(out_size):
+        center = (o + 0.5) * scale
+        lo = max(int(center - support + 0.5), 0)
+        n = min(int(center + support + 0.5), in_size) - lo
+        w = [max(0.0, 1.0 - abs((j + lo - center + 0.5) * ss)) for j in range(n)]
+        total = 0.0
+        for v in w:                            # sequential sum, as the C loop adds them
+            total += v
+        xmin[o] = lo
+        for j, v in enumerate(w):
+            taps[o, j] = int(0.5 + (v / total if total != 0.0 else v) * (1 << 22))
+        k = max(k, n)
+    return xmin, np.ascontiguousarray(taps[:, :k])     # the table stride is the widest run
+
+
+def resize_images(images_u8, img_wh, device=None):
+    """PIL.Image.resize(img_wh, Image.BILINEAR) of every image of a uint8 (N,H,W,3) RGB batch
+    (the network input of datasets/dtu.py:159-162, tanks.py, blendedmvs.py:162-163), bit-exact,
+    on the GPU by casmvs_resize_u8_fwd -> uint8 (N,h,w,3) CUDA tensor, (w, h) = img_wh.
+    `images_u8` may be a host tensor / ndarray (uploaded as bytes to `device`) or on the device.
+    Images that already have the size are returned as they are (on the device)."""
+    import ctypes
+
+    from . import _lib
+    t = images_u8 if torch.is_tensor(images_u8) else torch.from_numpy(np.ascontiguousarray(images_u8))
+    if t.dtype != torch.uint8 or t.dim() != 4 or t.shape[-1] != 3:
+        raise _lib.CasMVSError("resize_images expects uint8 (N,H,W,3)")
+    if not t.is_cuda:
+        if device is None:
+            raise _lib.CasMVSError("resize_images: give a CUDA device for host input (no CPU path)")
+        t = t.to(device, non_blocking=True)
+    t = t.contiguous()
+    N, H, W, _ = t.shape
+    w, h = int(img_wh[0]), int(img_wh[1])
+    if (w, h) == (W, H):
+        return t
+    out = torch.empty(N, h, w, 3, device=t.device, dtype=torch.uint8)
+
+    def tables(n_in, n_out):
+        if n_in == n_out:
+            return None, None, 0
+        xmin, taps = pil_bilinear_coeffs(n_in, n_out)
+        return (torch.from_numpy(xmin).to(t.device), torch.from_numpy(taps).to(t.device), taps.shape[1])
+    xmin_x, taps_x, kx = tables(W, w)
+    xmin_y, taps_y, ky = tables(H, h)
+
+    def p(x):
+        return ctypes.c_void_p(x.data_ptr()) if x is not None else None
+    with torch.cuda.device(t.device):
+        st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
+        _lib.check(_lib.load().casmvs_resize_u8_fwd(
+            p(t), N, H, W, p(out), h, w, p(xmin_x), p(taps_x), kx, p(xmin_y), p(taps_y), ky, st),
+            "resize_u8")
     return out
 
 

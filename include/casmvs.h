@@ -295,6 +295,19 @@ int casmvs_regress_bwd(const float* logits, const float* depth_values, int dv_is
 int casmvs_normalize_u8_fwd(const uint8_t* images, float* out, int N, int H, int W,
                             const float* mean3, const float* std3, void* stream);
 
+/* PIL.Image.resize(size, Image.BILINEAR) of the same data sets (datasets/dtu.py:159-162,
+ * tanks.py, blendedmvs.py:162-163), bit-exact: in (N,H,W,3) uint8 RGB -> out (N,h,w,3) uint8.
+ * The taps are PIL's fixed-point coefficients, built on the host (io.pil_bilinear_coeffs):
+ * per output column x, xmin_x[x] and taps_x[x*kx .. x*kx+kx) int32 weights with 22 fractional
+ * bits (unused trailing taps 0); the same for rows.  All four tables are DEVICE arrays.  The
+ * horizontal pass runs first and is clipped to uint8, then the vertical pass; a pass whose
+ * axis keeps its size is skipped and its tables are ignored (may be NULL).  Returns an error
+ * when the taps of one 16x64 output tile do not fit shared memory (a 48 KB budget; the data
+ * sets need at most 4 taps per axis).  in and out must not overlap. */
+int casmvs_resize_u8_fwd(const uint8_t* in, int N, int H, int W, uint8_t* out, int h, int w,
+                         const int* xmin_x, const int* taps_x, int kx, const int* xmin_y,
+                         const int* taps_y, int ky, void* stream);
+
 /* ---- geometric-consistency filter + refinement + back-projection (SURVEY.md 8 f-3) ------
  * One reference view of eval.py:262-318 on the device; replaces xy_ref2src / xy_src2ref /
  * check_geo_consistency (eval.py:113-182, numba + cv2.remap on the CPU).  For every reference

@@ -106,7 +106,7 @@ extern "C" int casmvs_conv3d_fwd(const float* x, const float* w_packed, const fl
     if (rc <= 0) return rc;
     if (kind != CASMVS_CONV_PLANAR) {
       rc = conv3d_tma2(x, w_packed, scale, shift, slope, skip, y, B, Cin, Cout, D, h, w, kind,
-                       stride, precision, st);
+                       stride, pf, st);
       if (rc <= 0) return rc;
     }
     // no tensor-core kernel covers this layer shape: it runs on the CUDA cores (same TF32-rounded

@@ -522,7 +522,8 @@ static int launch2(const float* x, const float* wpk, Params p, cudaStream_t st) 
 // Returns 0 when handled, 1 when the layer shape is left to the other kernels.
 int conv3d_tma2(const float* x, const float* wpk, const float* scale, const float* shift,
                 float slope, const float* skip, float* y, int B, int Cin, int Cout, int D, int h,
-                int w, int kind, int stride, int precision, cudaStream_t st) {
+                int w, int kind, int stride, int precision_flags, cudaStream_t st) {
+  const int precision = precision_flags & 0xff;
   static int enabled = -1;
   if (enabled < 0) {
     const char* e = getenv("CASMVS_TMA2");
@@ -532,7 +533,9 @@ int conv3d_tma2(const float* x, const float* wpk, const float* scale, const floa
   if ((reinterpret_cast<uintptr_t>(x) & 15) != 0) return 1;
   tma2::Params p;
   p.scale = scale; p.shift = shift; p.skip = skip; p.y = y;
-  p.slope = slope; p.B = B; p.Di = D; p.Hi = h; p.Wi = w; p.Cout = Cout; p.round_out = 1;
+  p.slope = slope; p.B = B; p.Di = D; p.Hi = h; p.Wi = w; p.Cout = Cout;
+  // every layer this kernel covers has Cout > 1: stored rounded unless the caller asks for fp32
+  p.round_out = (precision_flags & CASMVS_KEEP_FP32_OUT) ? 0 : 1;
   if (kind == CASMVS_CONV && stride == 2 && (enabled & 1)) {
     if (skip) return 1;
     p.Do = (D - 1) / 2 + 1; p.Ho = (h - 1) / 2 + 1; p.Wo = (w - 1) / 2 + 1;

@@ -121,8 +121,11 @@ class FeatureNet(nn.Module):
 
         w0, b0, _, _, slope0 = cache[0]
         t = ops.conv2d_rgb8(x, w0, b0, slope0, round_tf32=True)
-        c0 = planar(t, 1, True)                       # consumers: cuDNN conv + lateral (fp32)
-        c1 = planar(planar(strided(c0, 2), 3, False), 4, True)
+        # c0 and c1 feed the next 5x5 stride-2 tcgen05 conv, which reads its operand by
+        # truncation: stored rounded to nearest (the fp32 lateral merges then read a value within
+        # half a TF32 ulp, unbiased).  c2 is read by the fp32 toplayer merge only.
+        c0 = planar(t, 1, False)
+        c1 = planar(planar(strided(c0, 2), 3, False), 4, False)
         c2 = planar(planar(strided(c1, 5), 6, False), 7, True)
         f2 = ops.fpn_merge(None, c2, self.toplayer.weight, self.toplayer.bias)
 
